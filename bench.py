@@ -24,6 +24,10 @@ against oracle/_ref on a seeded random sample of THIS rank's outputs (every rank
            issue rate measured live by a microkernel; plus the (non-binding) HBM view.
 `cpu_baseline`: the unmodified reference (oracle/_ref) on the host cores, bounded sample, whose
            outputs are also compared byte-for-byte with the GPU's.
+
+--dump-outputs DIR writes each config's outputs of its last timed step to DIR/<config>.npy (see
+dump_outputs); the inputs depend only on the arguments, so two builds of the library can be
+compared output for output.
 """
 from __future__ import annotations
 import argparse
@@ -363,6 +367,29 @@ def sample_indices(n, m, seed):
     return np.sort(np.concatenate([body.astype(np.int64), np.arange(n - tail, n, dtype=np.int64)]))
 
 
+DUMP_BYTES = 60 << 20          # --dump-outputs: every .npy file of one run, all ranks together, stays below 64 * 10^6 bytes
+
+
+def dump_rows(n, gt, n_configs, world):
+    """outputs per config and rank that --dump-outputs writes: all n if they fit the share of
+    DUMP_BYTES of one config on one of the world ranks, at one float32 per wire byte, else a
+    sample of that size"""
+    return max(1, min(n, DUMP_BYTES // (n_configs * world) // (4 * gt)))
+
+
+def dump_outputs(out_dir, wname, dO, n, gt, m, rank, world):
+    """out_dir/<config>.npy (<config>.rank<r>.npy on more than one rank): the GT elements of m
+    seeded outputs of this rank's batch (sample_indices; all of them when m == n), one row per
+    output, one float32 per wire byte (exact).  The same arguments give the same rows every run."""
+    import numpy as np
+    import torch
+    idx = torch.from_numpy(sample_indices(n, m, SEED + rank)).to(dO.device)
+    rows = dO.view(n, gt).index_select(0, idx).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    name = wname if world == 1 else "%s.rank%d" % (wname, rank)
+    np.save(os.path.join(out_dir, name + ".npy"), rows.astype(np.float32))
+
+
 def cpu_sample(wname, w, Ph, Qh, n, rank, world, seconds, want_cpu):
     """run the reference on a seeded sample of this rank's outputs (before CUDA is initialised: the
     workers fork).  Returns (idx, expected bytes, cpu_baseline dict)."""
@@ -467,9 +494,10 @@ class GpuRun:
         return self.peak
 
 
-def run_config(G, wname, args, Ph, Qh, n, idx, cpu_out, cpu, steps, warmup, per_step_flush):
+def run_config(G, wname, args, Ph, Qh, n, idx, cpu_out, cpu, steps, warmup, per_step_flush, dump_m=0):
     """time one workload on this process's GPU (all ranks call it together).  Returns the config's
-    record on rank 0 (None elsewhere)."""
+    record on rank 0 (None elsewhere).  With args.dump_outputs, dump_m outputs of the last timed
+    step go to that directory (dump_outputs)."""
     import numpy as np
     from pbc_b200.pairing import Pairing, kernel_launches
     torch = G.torch
@@ -533,6 +561,8 @@ def run_config(G, wname, args, Ph, Qh, n, idx, cpu_out, cpu, steps, warmup, per_
         torch.cuda.synchronize()
         ms_total = e0.elapsed_time(e1)
     launches = kernel_launches() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, wname, dO, n, gt, dump_m, G.rank, world)
     G.barrier()
     # per-kernel durations: CUDA events recorded by the library on the launching stream
     stage = [0.0, 0.0, 0.0]
@@ -709,8 +739,17 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=0.0, help="CPU parity/baseline budget per config (default: per-config table)")
     ap.add_argument("--ref-seconds", type=float, default=3.0, help="--impl reference: seconds per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--extra-steps", type=int, default=5, help="timed steps of each extra config")
+    ap.add_argument("--extra-steps", type=int, default=None, help="timed steps of each extra config (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write each config's outputs of its last timed step to DIR/<config>.npy "
+                         "(<config>.rank<r>.npy per rank on more than one GPU; float32, one row per output, one column "
+                         "per wire byte; a fixed seeded sample where all of them would exceed 64 MB over all files of "
+                         "all ranks)")
     args = ap.parse_args()
+    if args.steps < 1 or (args.extra_steps is not None and args.extra_steps < 1):
+        ap.error("--steps and --extra-steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl b200)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -748,12 +787,13 @@ def main():
     recs = {}
     for i, wname in enumerate(names):
         Ph, Qh, n, idx, cpu_out, cpu = plans.pop(wname)
+        dump_m = dump_rows(n, WIRE[WORKLOADS[wname]["param"]][2], len(names), world)
         if i == 0:
-            recs[wname] = run_config(G, wname, args, Ph, Qh, n, idx, cpu_out, cpu, args.steps, args.warmup, False)
+            recs[wname] = run_config(G, wname, args, Ph, Qh, n, idx, cpu_out, cpu, args.steps, args.warmup, False, dump_m)
         else:
             try:
                 recs[wname] = run_config(G, wname, args, Ph, Qh, n, idx, cpu_out, cpu,
-                                         max(1, min(args.steps, args.extra_steps)), 3, True)
+                                         args.extra_steps or args.steps, 3, True, dump_m)
             except Exception as e:                  # noqa: BLE001
                 recs[wname] = {"error": str(e)[:300]}
         del Ph, Qh
